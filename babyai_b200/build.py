@@ -1,12 +1,14 @@
 """Builds babyai_b200/libbabyai_b200.so (the C-ABI library of include/babyai_b200.h)
 from babyai_b200/csrc/pool.cu with nvcc for sm_100a, in-tree."""
+import glob
 import os
 import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, 'csrc', 'pool.cu')
-DEPS = [SRC, os.path.join(HERE, 'csrc', 'env_logic.cuh'), os.path.join(HERE, 'csrc', 'level_params.h'), os.path.join(HERE, 'csrc', 'simt.cuh'), os.path.join(HERE, 'csrc', 'gen_round.cuh'), os.path.join(HERE, 'csrc', 'rollout_lane.cuh'), os.path.join(HERE, 'csrc', 'rollout_cta.cuh'), os.path.join(HERE, 'csrc', 'rgb_tiles.h'), os.path.join(HERE, '..', 'include', 'babyai_b200.h')]
+# every source the library is compiled from: a change to any of them rebuilds it
+DEPS = sorted(glob.glob(os.path.join(HERE, 'csrc', '*'))) + [os.path.join(HERE, '..', 'include', 'babyai_b200.h')]
 OUT = os.path.join(HERE, 'libbabyai_b200.so')
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec of the batched BabyAI pool (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--level L] [--envs E]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--level L] [--envs E] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- BabyAI-GoToLocal-v0,
 65 536 environments per GPU, uniform random actions, ParallelEnv auto-reset on.
@@ -11,10 +11,9 @@ Own arm, printed as ONE JSON line by rank 0:
   value     env-steps/sec, whole job, actions resident in HBM ([T, N] int8),
             observations written to a [T, N, 147] rollout buffer (385 MB > L2).
             The timed region is ALWAYS calls of bb_pool_rollout (the persistent
-            stepping kernel, T = 40 steps per launch): K is rounded up to whole
-            rollouts and to at least MIN_TIMED_STEPS steps (`steps` = what was timed,
-            `steps_requested` = K); CUDA events, barrier + synchronize on both
-            sides, max over ranks.
+            stepping kernel, T = 40 steps per launch) covering exactly K steps:
+            K // T whole rollouts and one of K % T steps; CUDA events, barrier +
+            synchronize on both sides, max over ranks.
   roofline  achieved = 153 algorithmic bytes per env-step (147 obs + 4 reward +
             1 done + 1 action; SURVEY.md 8d) x the per-GPU `value` of that SAME
             timed region, against MEASURED_PEAKS.json hbm_gbs; `kernel_frac` is
@@ -48,7 +47,6 @@ sys.path.insert(0, ROOT)
 LEVEL = 'GoToLocal'
 N_ENVS = 65536
 CHUNK = int(os.environ.get("BENCH_CHUNK", "40"))   # rollout length per launch (= --frames-per-proc, arguments.py:42)
-MIN_TIMED_STEPS = 1000          # the timed region never covers fewer steps than this (25 launches of 40 steps)
 MIN_HOST_STEPS = 200            # ... and the per-step legs (e2e, per_step_api) never fewer than this
 ALGO_BYTES_PER_STEP = 153       # 147 obs + 4 reward + 1 done + 1 action (SURVEY.md 8d)
 FALLBACK_HBM_GBS = 6650.0       # /opt/skills/guides/B200_PROFILING.md fallback
@@ -209,6 +207,20 @@ def run_reference(args, rank):
     print(json.dumps(out), flush=True)
 
 
+def write_outputs(out_dir, arrays, limit=64 << 20):
+    """arrays: name -> float32 array whose first axis is the environment.  Writes out_dir/<name>.npy; when all of them
+    together exceed `limit` bytes, only a fixed, seeded sample of environments (listed in env_index.npy)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(arrays['reward'])
+    per_env = sum(a.nbytes for a in arrays.values()) // n
+    if n * per_env > limit:
+        idx = np.sort(np.random.RandomState(0).choice(n, (limit - 4096) // (per_env + 8), replace=False))
+        arrays = dict({k: a[idx] for k, a in arrays.items()}, env_index=idx.astype(np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -221,7 +233,11 @@ def main():
     ap.add_argument('--brief', action='store_true', help='device-resident value + kernel timing only (child runs of --other-configs)')
     ap.add_argument('--lean', action='store_true', help='value, roofline and e2e only (multi-GPU scaling runs of the other configs)')
     ap.add_argument('--no-other-configs', action='store_true', help='skip the child runs of BASELINE configs 3-5 (per-GPU share)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step returned to rank 0 (obs, reward, done, '
+                                                          'direction) as DIR/<name>.npy, float32')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
 
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -275,13 +291,15 @@ def main():
     done = torch.empty((T, n), dtype=torch.uint8, device=dev)
     dirs = torch.empty((T, n), dtype=torch.int8, device=dev)
 
-    def run_rollouts(r):
-        for _ in range(r):
-            env.rollout(actions, obs, rew, done, dirs)
+    bufs = (actions, obs, rew, done, dirs)
 
-    # ---- device-resident throughput: whole rollouts, whatever K ---------------------------------
-    n_roll = max((K + T - 1) // T, (MIN_TIMED_STEPS + T - 1) // T)
-    K_eff = n_roll * T
+    def run_rollouts(r, bufs=bufs):
+        for _ in range(r):
+            env.rollout(*bufs)
+
+    # ---- device-resident throughput: exactly K steps, K // T whole rollouts and one of K % T steps ----
+    n_roll, K_rest = divmod(K, T)
+    rest_bufs = [b[:K_rest] for b in bufs]
     w_roll = max((max(W, 3) + T - 1) // T, 2)
     run_rollouts(w_roll)
     barrier()
@@ -293,10 +311,16 @@ def main():
     barrier()
     e0.record()
     run_rollouts(n_roll)
+    if K_rest:
+        run_rollouts(1, rest_bufs)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = env.launches() - l0
+    if args.dump_outputs and rank == 0:
+        last = (K_rest or T) - 1
+        dump = {'obs': obs[last], 'reward': rew[last], 'done': done[last], 'direction': dirs[last]}
+        dump = {k: v.cpu().numpy().astype(np.float32) for k, v in dump.items()}
     # keep the GPU busy a little longer so the clock sampler sees load even for short K
     clocks = None
     if rank == 0:
@@ -318,12 +342,14 @@ def main():
     k_refill_ms = sum(kf) / len(kf) if kf else 0.0      # amortised per launch
 
     peak, peak_src = hbm_peak()
-    value = world * n * K_eff / (ms * 1e-3)
+    value = world * n * K / (ms * 1e-3)
     achieved = ALGO_BYTES_PER_STEP * (value / world) / 1e9           # GB/s of algorithmic bytes per GPU, SAME timed region
     kernel_achieved = ALGO_BYTES_PER_STEP * n * T / (k_roll_ms * 1e-3) / 1e9 if k_roll_ms > 0 else 0.0
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, dump)
     if args.brief:
         if rank == 0:
-            print(json.dumps({'level': args.level, 'envs_per_gpu': n, 'value': value, 'us_per_step': 1e3 * ms / K_eff, 'steps': K_eff,
+            print(json.dumps({'level': args.level, 'envs_per_gpu': n, 'value': value, 'us_per_step': 1e3 * ms / K, 'steps': K,
                               'kernel_us_per_step': 1e3 * k_roll_ms / T, 'refill_ms_per_launch': k_refill_ms,
                               'roofline_frac': achieved / peak, 'counters': env.counters()}), flush=True)
         if world > 1:
@@ -473,16 +499,15 @@ def main():
             except Exception:
                 traffic = None
         out = {
-            'metric': METRIC, 'value': value, 'unit': 'env-steps/s', 'n_gpus': world, 'steps': K_eff, 'steps_requested': K,
-            'warmup': w_roll * T, 'ms_per_step': ms / K_eff, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
+            'metric': METRIC, 'value': value, 'unit': 'env-steps/s', 'n_gpus': world, 'steps': K, 'steps_requested': K,
+            'warmup': w_roll * T, 'ms_per_step': ms / K, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
             'dtype': 'u8', 'data': 'synthetic',
             'config': {'workload': workload(args.level, n),
                        'envs_per_gpu': n, 'rollout_chunk': T,
                        'l2_policy': 'obs written to a [%d, %d, 147] buffer (%.0f MB) larger than L2' % (T, n, T * n * 147 / 1e6),
-                       'execution': 'timed region = %d calls of bb_pool_rollout (%d steps each; K = %d requested, rounded up to whole '
-                                    'rollouts and to >= %d steps): one persistent stepping kernel per call with the env state resident in '
-                                    'shared memory; level generation inside it (single-room levels) or beside it on a side stream' %
-                                    (n_roll, T, K, MIN_TIMED_STEPS),
+                       'execution': 'timed region = %d calls of bb_pool_rollout (%d steps each) and %d of %d steps: one persistent '
+                                    'stepping kernel per call with the env state resident in shared memory; level generation inside it '
+                                    '(single-room levels) or beside it on a side stream' % (n_roll, T, 1 if K_rest else 0, K_rest),
                        'actions': 'int8 [T, N], resident in HBM',
                        'parallelism': 'replicas x%d, counters all-gather only' % world,
                        'numa': numa},

@@ -7,7 +7,7 @@ import numpy as np
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 CONFIG_LEVELS = ['GoToRedBall', 'GoToLocal', 'PickupLoc', 'GoTo', 'BossLevel']
-GOLDEN_LEVELS = sorted(f[:-4] for f in os.listdir(GOLDEN) if f.endswith('.npz') and not f.startswith(('succ_', 'rgb_', 'done_', 'bonus_')))      # all 47 served levels (CPU replays)
+GOLDEN_LEVELS = sorted(f[:-4] for f in os.listdir(GOLDEN) if f.endswith('.npz') and not f.startswith(('succ_', 'rgb_', 'done_', 'bonus_', 'ref_')))      # all 47 served levels (CPU replays)
 # success-heavy reference traces (97 % bot actions, >= 50 successful episodes each; make_golden.py --success): 'succ_<Level>'
 # reference traces generated with BABYAI_DONE_ACTIONS=1 (verifier.use_done_actions; make_golden.py --done-actions): 'done_<Level>'
 DONE_GOLDENS = sorted(f[:-4] for f in os.listdir(GOLDEN) if f.endswith('.npz') and f.startswith('done_'))
@@ -19,6 +19,52 @@ SUCCESS_GOLDENS = sorted(f[:-4] for f in os.listdir(GOLDEN) if f.endswith('.npz'
 GOLDEN_LEVELS_GPU = ['BossLevel', 'BossLevelNoUnlock', 'GoTo', 'GoToLocal', 'GoToObjMazeS4R2', 'GoToOpen', 'GoToRedBall',
                      'GoToRedBallGrey', 'GoToSeq', 'MiniBossLevel', 'Open', 'Pickup', 'PickupLoc', 'PutNext', 'PutNextLocal',
                      'PutNextLocalS5N3', 'Synth', 'SynthSeq', 'UnblockPickup']
+
+
+REFERENCE_RUNS = os.path.join(GOLDEN, 'ref_runs.npz')
+BOT_HANGS = ('UnlockToUnlock', 'KeyInBox')                 # the reference's bot does not return on these (its search loops)
+
+
+def reference_runs():
+    """Every run of the reference's own level code that the step-by-step comparisons replay, as (group, level, arguments of
+    compare_ref.record); tests/golden/make_ref_golden.py records them into ref_runs.npz."""
+    from babyai_b200.levels import BONUS_LEVELS, ICLR19_LEVELS
+    runs = [('config_random', lv, dict(seed=4000 + s, steps=150, policy='random', act_seed=s)) for lv in CONFIG_LEVELS for s in range(2)]
+    runs += [('iclr_random', lv, dict(seed=7100 + 17 * s, steps=300, policy='random', act_seed=10 + s))
+             for lv in sorted(ICLR19_LEVELS) for s in range(3)]
+    runs += [('iclr_bot', lv, dict(seed=7300, steps=200, policy='bot', act_seed=3)) for lv in sorted(ICLR19_LEVELS)]
+    runs += [('bot', lv, dict(seed=5000, steps=250, policy='bot', act_seed=1))
+             for lv in ['GoToLocal', 'PickupLoc', 'BossLevel', 'SynthSeq', 'GoToImpUnlock', 'Unlock']]
+    for lv in BONUS_LEVELS:
+        # reset() of a *Carrying level hands back the pre-carry observation: the states differ until the first step
+        flags = dict(state_at_reset=not lv.endswith('Carrying'), check_draws=False)
+        runs += [('bonus', lv, dict(seed=300 + 7 * k, steps=160, policy='random', act_seed=k, **flags)) for k in range(3)]
+        if lv not in BOT_HANGS:
+            runs.append(('bonus', lv, dict(seed=900, steps=160, policy='bot', act_seed=5, **flags)))
+    return runs
+
+
+_recorded = {}
+
+
+def replay_reference_runs(group, level, make_pool=None):
+    """Replays the recorded reference runs of (group, level) on a one-env pool (compare_ref.replay); returns the number of
+    episodes that ended."""
+    import compare_ref
+    if not _recorded:                       # the runs are stored end to end (make_ref_golden.py runs())
+        z = np.load(REFERENCE_RUNS)
+        a = np.concatenate([[0], np.cumsum(z['steps'])])
+        c = np.concatenate([[0], np.cumsum((z['steps'] + compare_ref.EVERY - 1) // compare_ref.EVERY)])
+        for i, key in enumerate(json.loads(str(z['keys']))):
+            _recorded[key] = z['actions'][a[i]:a[i + 1]], z['checks'][c[i]:c[i + 1]]
+    runs = [kw for g, lv, kw in reference_runs() if (g, lv) == (group, level)]
+    assert runs, (group, level)
+    episodes = 0
+    for kw in runs:
+        actions, checks = _recorded[compare_ref.run_key(level, **kw)]
+        flags = {k: kw[k] for k in ('state_at_reset', 'check_draws') if k in kw}
+        episodes += compare_ref.replay(level, kw['seed'], actions, checks, make_pool=make_pool, **flags)
+    return episodes
 
 
 def load_golden(level):

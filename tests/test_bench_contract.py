@@ -36,3 +36,24 @@ def test_reference_arm_other_ranks_stay_silent():
                           '--warmup', '1'], capture_output=True, text=True, timeout=120,
                          env=dict(os.environ, RANK='1', LOCAL_RANK='1', WORLD_SIZE='2'))
     assert out.returncode == 0 and out.stdout.strip() == ''
+
+
+def test_dump_outputs_keeps_a_fixed_sample_under_the_cap(tmp_path):
+    """--dump-outputs writes at most 64 MB: a larger output is cut down to the same seeded sample of environments every time"""
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    from bench import write_outputs
+    n = 120000                                                   # 600 bytes per environment: 72 MB in all
+    arrays = {'obs': np.arange(n * 147, dtype=np.float32).reshape(n, 7, 7, 3), 'reward': np.arange(n, dtype=np.float32),
+              'done': np.zeros(n, np.float32), 'direction': np.ones(n, np.float32)}
+    for d in ('a', 'b'):
+        write_outputs(str(tmp_path / d), arrays)
+    files = sorted(os.listdir(str(tmp_path / 'a')))
+    assert files == ['direction.npy', 'done.npy', 'env_index.npy', 'obs.npy', 'reward.npy']
+    assert sum(os.path.getsize(str(tmp_path / 'a' / f)) for f in files) <= 64 << 20
+    idx = np.load(str(tmp_path / 'a' / 'env_index.npy'))
+    assert idx.dtype == np.float64 and np.array_equal(idx, np.load(str(tmp_path / 'b' / 'env_index.npy')))
+    assert np.array_equal(np.load(str(tmp_path / 'a' / 'reward.npy')), idx.astype(np.float32))
+    assert np.array_equal(np.load(str(tmp_path / 'a' / 'obs.npy')), arrays['obs'][idx.astype(np.int64)])
+    write_outputs(str(tmp_path / 'small'), {k: a[:1000] for k, a in arrays.items()})
+    assert sorted(os.listdir(str(tmp_path / 'small'))) == ['direction.npy', 'done.npy', 'obs.npy', 'reward.npy']

@@ -1,8 +1,9 @@
 """The 50 bonus levels (babyai/levels/bonus_levels.py) against the REFERENCE ITSELF: the reference's unmodified level classes
 on the gym_minigrid shim (Philox back-end), step by step against the host build of the kernel source (tests/hostemu) --
 observation, direction, mission, reward, done, every grid cell, agent pose, carried object, step counters and the number
-of RNG draws (oracle/compare_ref.py).  The C oracle does not cover these families: their checker is the reference directly
-(here, build container only) and the reference-generated traces under tests/golden/bonus_*.npz, which the CUDA pool replays."""
+of RNG draws (oracle/compare_ref.py), recorded from the reference into tests/golden/ref_runs.npz (make_ref_golden.py).  The
+C oracle does not cover these families: their checker is the reference's runs and the reference-generated traces under
+tests/golden/bonus_*.npz, which the CUDA pool replays."""
 import os
 import sys
 
@@ -14,9 +15,7 @@ for p in (ROOT, os.path.join(ROOT, 'oracle'), os.path.join(ROOT, 'tests', 'hoste
     if p not in sys.path:
         sys.path.insert(0, p)
 from babyai_b200.levels import BONUS_LEVELS, detokenize, level_spec  # noqa: E402
-
-
-BOT_HANGS = ('UnlockToUnlock', 'KeyInBox')                 # the reference's bot does not return on these (its search loops)
+from common import replay_reference_runs  # noqa: E402
 
 
 class _One(object):
@@ -41,14 +40,8 @@ class _One(object):
         return self.p.state(i)
 
 
-@pytest.mark.reference
 @pytest.mark.timeout(600)
 @pytest.mark.parametrize('level', BONUS_LEVELS)
 def test_bonus_level_equals_reference(level):
-    import compare_ref
-    carrying = level.endswith('Carrying')          # reset() hands back the pre-carry observation: the states differ until the first step
-    eps = 0
-    for k in range(3):
-        eps += compare_ref.compare(level, 300 + 7 * k, 160, 'random', act_seed=k, make_pool=_One, state_at_reset=not carrying, check_draws=False)
-    if level not in BOT_HANGS:
-        eps += compare_ref.compare(level, 900, 160, 'bot', act_seed=5, make_pool=_One, state_at_reset=not carrying, check_draws=False)
+    """3 random-action runs and (where the reference's bot returns) one bot-driven run per level"""
+    replay_reference_runs('bonus', level, make_pool=_One)

@@ -1,6 +1,7 @@
 """The demo wire format (scripts/make_agent_demos.py:116, babyai/utils/demos.py:38-64): demos built from batched frozen-at-done
-episodes must be what the reference's own one-env-at-a-time loop produces for the same seeds and actions, and must read
-back through the reference's `transform_demos`."""
+episodes must be what the reference's own one-env-at-a-time loop produces for the same seeds and actions (recorded in
+tests/golden/ref_demos.npz by make_ref_golden.py), tuple for tuple after a pickle round trip."""
+import json
 import os
 import pickle
 import sys
@@ -27,42 +28,34 @@ def _batched_episodes(level, seeds, acts):
     return missions, np.stack(imgs), np.stack(dirs), np.stack(dones), np.stack(rews)
 
 
-@pytest.mark.reference
-@pytest.mark.parametrize('level', ['GoToLocal', 'PickupLoc', 'GoToObjMazeS4R2'])
-def test_demos_equal_the_reference_loop(level):
-    import refenv
-    gym = refenv.setup('philox')
-    import blosc                                              # the shim's stand-in (oracle/shim/blosc.py)
-    from babyai.utils.demos import transform_demos
-    from babyai_b200.demos import episodes_to_demos
+DEMO_LEVELS = ['GoToLocal', 'PickupLoc', 'GoToObjMazeS4R2']
+
+
+def demo_actions():
+    """actions [T, n] and seeds of the demo comparison"""
     n, T, seed = 40, 150, 7000
     rng = np.random.RandomState(1)
     acts = rng.choice(7, size=(T, n), p=[0.15, 0.15, 0.45, 0.08, 0.05, 0.1, 0.02]).astype(np.int8)
-    seeds = [seed + k for k in range(n)]
+    return acts, [seed + k for k in range(n)]
+
+
+@pytest.mark.parametrize('level', DEMO_LEVELS)
+def test_demos_equal_the_reference_loop(level):
+    from babyai_b200.demos import episodes_to_demos
+    acts, seeds = demo_actions()
     missions, imgs, dirs, dones, rews = _batched_episodes(level, seeds, acts)
-    ours = episodes_to_demos(missions, imgs, dirs, acts, dones, rews, pack_array=blosc.pack_array)
+    ours = pickle.loads(pickle.dumps(episodes_to_demos(missions, imgs, dirs, acts, dones, rews, pack_array=pickle.dumps)))
     # the reference's loop (make_agent_demos.generate_demos), one env at a time, same seeds, same action streams
-    theirs = []
-    for k in range(n):
-        env = refenv.make_env(level, seeds[k], 'philox')
-        obs = env.reset()
-        mission, images, directions, actions = obs['mission'], [], [], []
-        done, reward, t = False, 0, 0
-        while not done and t < T:
-            a = int(acts[t, k])
-            new_obs, reward, done, _ = env.step(a)
-            actions.append(a); images.append(obs['image']); directions.append(obs['direction'])
-            obs = new_obs
-            t += 1
-        if done and reward > 0:
-            theirs.append((mission, blosc.pack_array(np.array(images)), directions, actions))
+    z = np.load(os.path.join(ROOT, 'tests', 'golden', 'ref_demos.npz'))
+    theirs = json.loads(str(z[level + '.missions']))
     assert len(ours) == len(theirs) > 0
-    a, b = transform_demos(pickle.loads(pickle.dumps(ours))), transform_demos(theirs)
-    for da, db in zip(a, b):
-        assert len(da) == len(db)
-        for (oa, aa, na), (ob, ab, nb) in zip(da, db):
-            assert np.array_equal(oa['image'], ob['image']) and oa['direction'] == ob['direction'] and oa['mission'] == ob['mission']
-            assert aa == ab and na == nb
+    t0 = 0
+    for (mission, packed, directions, actions), want in zip(ours, theirs):
+        t1 = t0 + len(actions)
+        assert mission == want and np.array_equal(pickle.loads(packed), z[level + '.images'][t0:t1])
+        assert list(directions) == z[level + '.directions'][t0:t1].tolist() and list(actions) == z[level + '.actions'][t0:t1].tolist()
+        t0 = t1
+    assert t0 == len(z[level + '.actions'])
 
 
 def test_unfinished_and_failed_episodes_are_dropped():

@@ -69,14 +69,41 @@ def test_own_arm_json_line():
     r = d['roofline']
     assert r['bound'] == 'hbm' and r['unit'] == 'GB/s' and r['achieved'] > 0 and abs(r['frac'] - r['achieved'] / r['peak']) < 1e-9
     assert d['e2e']['h2d_bytes_per_step'] == 4096 and d['e2e']['d2h_bytes_per_step'] == 4096 * 153
-    # the roofline comes from the SAME timed region as `value`, which always runs whole rollouts (never fewer than 1000 steps)
-    assert d['steps'] >= 1000 and d['steps'] % 40 == 0 and d['steps_requested'] == 80
+    # the roofline comes from the SAME timed region as `value`, which covers exactly the requested steps
+    assert d['steps'] == d['steps_requested'] == 80
     assert abs(d['value'] / d['n_gpus'] * 153 / 1e9 - r['achieved']) <= 1e-6 * r['achieved'] and r['kernel_frac'] > 0
     assert abs(d['ms_per_step'] * d['steps'] * 1e-3 * d['value'] - d['steps'] * 4096) <= 1e-3 * d['steps'] * 4096
     assert d['e2e']['steps'] >= 200 and d['per_step_api']['steps'] >= 200 and d['e2e']['per_rank']['min'] > 0
     assert d['reference_parallel_env']['available'] is False and d['facade_e2e']['value'] > 0
     assert d['gpu_launches'] > 0 and d['counters']['errors'] == 0 and d['dtype'] == 'u8'
     assert 'error' not in d['learner_path']['tensor_copies'] and 'error' not in d['learner_path']['fused_io'], d['learner_path']
+
+
+def test_own_arm_dumps_the_last_timed_step(tmp_path):
+    """--dump-outputs: the last of exactly --steps timed steps (here two whole rollouts of 40 and one of 10), the same on
+    every run, and equal to the C oracle stepped through the warm-up and the timed steps with the same seeds and actions"""
+    import torch
+    import oracle as orc
+    from test_bench_contract import _line
+    from babyai_b200.sharding import shard_seeds
+    n, T, warm, K = 4096, 40, 80, 90
+    outs = []
+    for k in range(2):
+        d = _line(['--lean', '--steps', str(K), '--warmup', '40', '--envs', str(n), '--no-cpu-baseline', '--no-other-configs',
+                   '--dump-outputs', str(tmp_path / str(k))])
+        assert d['steps'] == K and d['warmup'] == warm
+        outs.append({f: np.load(str(tmp_path / str(k) / (f + '.npy'))) for f in ('obs', 'reward', 'done', 'direction')})
+    assert all(a.dtype == np.float32 for a in outs[0].values()) and outs[0]['obs'].shape == (n, 7, 7, 3)
+    assert all(np.array_equal(outs[0][f], outs[1][f]) for f in outs[0])
+    acts = torch.randint(0, 7, (T, n), device='cuda', dtype=torch.int8,
+                         generator=torch.Generator(device='cuda').manual_seed(1234)).cpu().numpy()
+    ref = orc.OraclePool('GoToLocal', n, shard_seeds(1, n, 0, 1))
+    ref.reset()
+    for t in list(range(T)) * ((warm + K) // T) + list(range((warm + K) % T)):
+        o, r, dn = ref.step(acts[t], nthreads=16)
+    assert np.array_equal(outs[0]['obs'], o.astype(np.float32)) and np.array_equal(outs[0]['reward'], r)
+    assert np.array_equal(outs[0]['done'], dn.astype(np.float32))
+    assert np.array_equal(outs[0]['direction'], np.asarray(ref.direction, np.float32))
 
 
 # ---- from here on: kernels instantiated after the last GPU visit (k_gen<true>, k_step8<*, true>, k_rollout<1, true>) ----
